@@ -25,6 +25,10 @@ max-over-ranks time and the final waveform gather.
             oracle/_ref/ by __graft_entry__.build(); kind "reference") -- or, if it is absent, the oracle
             port of it (kind "port") -- timed on the host cores over a bounded number of samples, with the
             4 threads the reference ships (synthesis.py:37) and with all host cores.
+
+--dump-outputs DIR writes what the last timed step of each path returned, as float32 .npy files: waveform.npy (the
+device path, (N x U, T)), e2e_waveform.npy ((U, 1, T_up)) and config4_waveform.npy ((8, T)); the last two are rank 0's.
+Inputs and noise seeds depend only on the arguments, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -38,6 +42,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 CFG2 = dict(out_channels=30, layers=24, stacks=4, residual_channels=512, gate_channels=512,
@@ -205,6 +210,21 @@ def measured_peak():
         return 6650.0, "fallback (B200_PROFILING.md 6.65 TB/s)"
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(d, arrays):
+    """Write each tensor as d/<name>.npy in float32.  Each gets an equal share of DUMP_BYTES; a larger one is replaced
+    by a fixed, seeded sample of its elements (flattened, in index order), the same positions on every run."""
+    os.makedirs(d, exist_ok=True)
+    share = (DUMP_BYTES // len(arrays) - 4096) // 4         # elements, 4 KB left for the .npy header
+    for name, t in arrays.items():
+        a = t.detach().float().cpu().numpy()
+        if a.size > share:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, share, replace=False))]
+        np.save(os.path.join(d, name + ".npy"), a)
+
+
 def run_reference(args, rank, world):
     """--impl reference: the reference's CPU incremental_forward on the host cores, rank 0 only."""
     if rank != 0:
@@ -250,7 +270,11 @@ def main():
     ap.add_argument("--cpu-samples", type=int, default=2000)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-config4", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step of each path as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -323,8 +347,10 @@ def main():
                              launches=eng.plan(U)["launches"] - launches0)
         if name == "device":
             wave_dev = out                       # (U, T) fp32 on this rank's GPU
+        else:
+            wave_e2e = out                       # (U, 1, T_up) fp32 on the host
     # BASELINE config 4's per-GPU share: 8 independent utterances in one launch
-    cfg4 = None
+    cfg4 = wave4 = None
     if not args.no_config4:
         U4, K4 = 8, max(1, min(K, 3))
         c4 = c_dev[:1].expand(U4, -1, -1).contiguous() if U < U4 else c_dev[:U4]
@@ -341,7 +367,7 @@ def main():
         barrier()
         e0.record()
         for i in range(K4):
-            step4(200 + i, False)
+            wave4 = step4(200 + i, False)
         e1.record()
         barrier()
         if conc:
@@ -364,6 +390,11 @@ def main():
         torch.cuda.synchronize(dev)
 
     if rank == 0:
+        if args.dump_outputs:
+            outs = {"waveform": torch.cat(gathered) if dist is not None else wave_dev, "e2e_waveform": wave_e2e}
+            if wave4 is not None:
+                outs["config4_waveform"] = wave4
+            dump_outputs(args.dump_outputs, outs)
         d, e = results["device"], results["e2e"]
         sps = d["samples"] / (d["ms"] * 1e-3)
         e_sps = e["samples"] / (e["ms"] * 1e-3)

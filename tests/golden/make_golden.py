@@ -1,19 +1,21 @@
 # coding: utf-8
 """Generate the golden vectors under tests/golden/ by running the UNMODIFIED reference.
 
-Run in the build container only (needs /root/reference):
+Needs a checkout of the original r9y9/wavenet_vocoder project:
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <path of the wavenet_vocoder checkout>
 
 For each small case it builds the reference ``WaveNet`` with seeded random weights, runs
   (1) teacher-forced ``incremental_forward`` while spying on the sampler input (the per-step head
       output the public API never returns for scalar-input models, SURVEY.md 8(c) recipe 1),
   (2) the batch ``forward()`` for the reference's own online==offline check
-      (tests/test_model.py:330-366), and
-  (3) free-running seeded ``incremental_forward``,
+      (tests/test_model.py:330-366),
+  (3) free-running seeded ``incremental_forward``, and
+  (4) the same over at most 48 steps with another torch seed,
 then runs oracle/wavenet_oracle.py on the same weights/inputs/seed, asserts BIT equality with the
-reference for (1) and (3), and writes everything to ``<case>.npz``.  The committed vectors let the
-oracle and the CUDA path be checked where /root/reference does not exist.
+reference for (1), (3) and (4), and writes (1)-(3) to ``<case>.npz`` and (4) of every case to
+``reference_arm.npz``.  The committed vectors let the oracle and the CUDA path be checked without
+the original project.
 """
 import os
 import sys
@@ -25,7 +27,9 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-sys.path.insert(0, "/root/reference")
+if len(sys.argv) != 2:
+    sys.exit("usage: python tests/golden/make_golden.py <path of the wavenet_vocoder checkout>")
+sys.path.insert(0, os.path.abspath(sys.argv[1]))
 warnings.filterwarnings("ignore")
 
 import wavenet_vocoder as ref_pkg                      # noqa: E402  (the reference)
@@ -62,6 +66,7 @@ CASES = {
                 output_distribution="Normal", dropout=0.0),
         B=2, T=48),
 }
+SHORT_SEED = 11
 
 
 def path_config(kw):
@@ -187,6 +192,16 @@ def make_case(name, spec):
                                              params_out=rec2)
         assert torch.equal(y_free_ref, y_free_rep), name
         params_free = torch.stack(rec2, dim=-1)
+        # (4) free running over at most 48 steps, another seed (the upsample network fixes the length)
+        upsample = kw.get("upsample_conditional_features", False)
+        T_short = T if upsample else min(T, 48)
+        torch.manual_seed(SHORT_SEED)
+        y_short_ref = model.incremental_forward(c=c_raw if c_raw is None or upsample else c_raw[..., :T_short],
+                                                g=g_ids, T=T_short)
+        torch.manual_seed(SHORT_SEED)
+        y_short_orc = orc.incremental_forward(cfg, w, c=None if c_up is None else c_up[..., :T_short], g=g_vec,
+                                              T=T_short)
+        assert torch.equal(y_short_ref, y_short_orc), name
 
     out.update({"sd." + k: v.numpy() for k, v in sd.items()})
     out.update({"noise." + k: v.numpy() for k, v in noise.items()})
@@ -213,6 +228,7 @@ def make_case(name, spec):
     np.savez_compressed(os.path.join(HERE, name + ".npz"), **out)
     print("%-14s ok  online/offline maxdiff %.2e  |y_free| mean %.3f" %
           (name, diff, float(np.abs(out["y_free"]).mean())))
+    return y_short_ref.numpy()
 
 
 def main():
@@ -222,8 +238,8 @@ def main():
     assert ref_pkg.receptive_field_size(12, 2, 3) == orc.receptive_field_size(12, 2, 3) == 253
     assert ref_pkg.receptive_field_size(30, 1, 3, dilation=lambda x: 1) == \
         orc.receptive_field_size(30, 1, 3, dilation=lambda x: 1) == 61
-    for name, spec in CASES.items():
-        make_case(name, spec)
+    short = {name: make_case(name, spec) for name, spec in CASES.items()}
+    np.savez_compressed(os.path.join(HERE, "reference_arm.npz"), seed=SHORT_SEED, **short)
 
 
 if __name__ == "__main__":
